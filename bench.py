@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--workload dense|hybrid|rerank|bm25] [--batch B] [--inner R] [--n-docs N] [--dim D] [--top-k K]
-                    [--rerank-k K2] [--shard auto|corpus|queries] [--no-extras]
+                    [--rerank-k K2] [--shard auto|corpus|queries] [--no-extras] [--dump-outputs DIR]
 
 Headline (`value`, `e2e`, `roofline`, `cpu_baseline`) = BASELINE.json configs[1]: 1 M docs x 1024-d, dense-only cosine
 top_k=100 on 1 x B200.  A STEP = `--inner` R batches of `--batch` B queries per GPU through the hot path (defaults 64 x 256
@@ -24,6 +24,10 @@ memory budget, 1 for the 2 GB corpus of the metric -> replicas, no collective). 
 value   : whole-job queries/sec, inputs already resident in HBM (device entry points, CUDA-event timed, max over ranks)
 e2e     : the same metric through the host-buffer C-ABI entry point (host queries -> H2D -> kernels -> D2H results)
 roofline: dominant kernel (the dense scan) algorithmic bytes / CUDA-event duration vs MEASURED_PEAKS.json hbm_gbs
+--dump-outputs DIR: after the timed steps, the headline leg's results of its LAST timed step (every batch of it, in order;
+          rank 0) as DIR/<name>.npy, float64 (ids and counts are exact integers), at most 64 MB in all (larger outputs:
+          a fixed, seeded sample of query rows, listed in DIR/query_rows.npy).  Inputs are seeded, so two builds run
+          with the same arguments can be compared array for array.
 cpu_baseline / --impl reference: the reference's CPU path (exact cosine in NumPy: fp32 `X @ q` with BLAS on a stated
           number of host threads + the best-first cut, both as the code base writes it -- full np.argsort,
           sparse.py:180 -- and with np.argpartition; BM25 via the rank_bm25 restatement) on a bounded sample.
@@ -54,6 +58,9 @@ METRIC = "retrieval queries/sec @1M docs,1024-d,top_k=100"  # BASELINE.json metr
 UNIT = "queries/s"
 DEFAULT_BATCH = {"dense": 256, "hybrid": 128, "rerank": 64, "bm25": 256}
 DEFAULT_INNER = {"dense": 64, "hybrid": 32, "rerank": 2, "bm25": 64}
+OUTPUT_NAMES = {"dense": ("ids", "scores", "counts"), "bm25": ("ids", "scores", "counts"),
+                "hybrid": ("ids", "scores", "sources", "counts"), "rerank": ("ids", "scores", "counts")}
+DUMP_LIMIT_BYTES = 64 << 20
 NAMES = {"dense": "dense-only cosine", "hybrid": "hybrid dense+BM25 rrf", "bm25": "BM25-only",
          "rerank": "hybrid dense+BM25 rrf + cross-encoder rerank (MiniLM-L6 random-init)"}
 
@@ -61,7 +68,7 @@ NAMES = {"dense": "dense-only cosine", "hybrid": "hybrid dense+BM25 rrf", "bm25"
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of every leg (the headline and each extra)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="dense", choices=["dense", "hybrid", "rerank", "bm25"])
@@ -85,7 +92,12 @@ def parse_args():
     ap.add_argument("--corpus-shards", type=int, default=0, help="explicit C (must divide N); overrides --shard")
     ap.add_argument("--gpu-mem-budget-gb", type=float, default=64.0,
                     help="HBM one GPU may spend on index data under --shard auto (B200: 180 GB)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the headline leg's results of its last timed step to DIR/<name>.npy (<= 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def peaks():
@@ -126,6 +138,7 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         time.sleep(0.15)
         self.proc.terminate()
+        self.proc.wait()
         sm, mx, pw, reasons = [], [], [], set()
         for ln in self.lines:
             f = [x.strip() for x in ln.split(",")]
@@ -386,7 +399,8 @@ class Leg:
         return float(t.item())
 
     # ---- the two timed regions
-    def run(self, steps, warmup, sample_clocks=True):
+    def run(self, steps, warmup, sample_clocks=True, capture=False):
+        """``capture``: also keep every batch result of the last timed step (device copies, ``outputs``)."""
         torch, eng = self.torch, self.eng
         inputs = [self.dev_inputs(j) for j in range(self.ring)]
         for s in range(warmup):
@@ -401,15 +415,23 @@ class Leg:
         if self.rank == 0 and sample_clocks:
             sampler.start()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        self.barrier()
-        ev0.record()
-        for s in range(steps):
-            for r in range(self.inner):
-                self.run_dev(inputs[(s * self.inner + r) % self.ring])
-        ev1.record()
-        self.barrier()
+        outputs = None
+        try:
+            self.barrier()
+            ev0.record()
+            for s in range(steps):
+                for r in range(self.inner):
+                    out = self.run_dev(inputs[(s * self.inner + r) % self.ring])
+                    if capture and s == steps - 1:   # the path reuses its output buffers: copy each batch aside
+                        if outputs is None:
+                            outputs = [torch.empty((self.inner, *t.shape), dtype=t.dtype, device=t.device) for t in out]
+                        for o, t in zip(outputs, out):
+                            o[r].copy_(t)
+            ev1.record()
+            self.barrier()
+        finally:
+            clocks = sampler.stop() if (self.rank == 0 and sample_clocks) else None
         ms_total = ev0.elapsed_time(ev1)
-        clocks = sampler.stop() if (self.rank == 0 and sample_clocks) else None
         launches = eng.launch_count() - launches0
         prof = {name: eng.profile_read(name) for name in ("dense_scan", "dense_merge", "dense_sample", "bm25_score",
                                                           "bm25_select", "fuse", "ce")}
@@ -461,7 +483,7 @@ class Leg:
                                if self.host_out else "pageable NumPy arrays (staged through the library's pinned buffers)"}
         return {"value": value, "ms_total": ms_total, "ms_per_step": ms_total / steps, "steps": steps, "n_batches": n_batches,
                 "clocks": clocks, "launches": int(launches), "prof": prof, "ce_stats": ce_stats, "e2e": e2e,
-                "timed_region_s": ms_total / 1e3}
+                "timed_region_s": ms_total / 1e3, "outputs": outputs}
 
     # ---- rooflines
     def roofline_dense(self, res):
@@ -597,6 +619,26 @@ def latency_b1(pipe, wl: Workload, idx, n_queries=200, top_k=100):
     return out
 
 
+def dump_outputs(path, kind, outputs):
+    """The last timed step's results as <path>/<name>.npy: [batches_per_step * queries_per_batch, ...] rows in the order
+    the step ran them, float64 (float32 arrays stay float32).  Above DUMP_LIMIT_BYTES a fixed, seeded sample of rows is
+    kept and its row numbers go to query_rows.npy."""
+    arrays = []
+    for name, t in zip(OUTPUT_NAMES[kind], outputs):
+        a = t.cpu().numpy()
+        a = a.reshape(-1, *a.shape[2:])
+        arrays.append((name, a if a.dtype == np.float32 else a.astype(np.float64)))
+    rows = arrays[0][1].shape[0]
+    row_bytes = sum(a.nbytes for _, a in arrays) // max(rows, 1)
+    if rows * row_bytes > DUMP_LIMIT_BYTES - (1 << 20):
+        keep = (DUMP_LIMIT_BYTES - (1 << 20)) // (row_bytes + 8)
+        sel = np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+        arrays = [(name, a[sel]) for name, a in arrays] + [("query_rows", sel.astype(np.float64))]
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays:
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 # --------------------------------------------------------------------------------------------- main
 _RESULT_OUT = sys.stdout
 
@@ -643,6 +685,8 @@ def main():
               "query_set": "1024 seeded unit vectors, cycled"}
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the results of the GPU path: use it with --impl b200")
         if rank != 0:
             return 0
         wl = Workload(args.n_docs, args.dim)
@@ -736,7 +780,10 @@ def main():
     idx = need_bm25(pipe, C, lo, hi) if kind in ("hybrid", "rerank", "bm25") else None
     rr = need_rerank(pipe, C, lo, hi) if kind == "rerank" else None
     leg = Leg(kind, pipe, wl, args, world, rank, local_rank, C, my_group, lo, hi, idx, rr)
-    res = leg.run(args.steps, args.warmup)
+    res = leg.run(args.steps, args.warmup, capture=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, kind, res["outputs"])
+    res["outputs"] = None
     roofline = leg.roofline_dense(res) if kind != "bm25" else {}
     if kind in ("hybrid", "rerank", "bm25"):
         roofline["bm25"] = leg.roofline_bm25(res)
@@ -745,7 +792,7 @@ def main():
 
     extras = set() if (args.no_extras or kind != "dense" or args.n_docs > 2_000_000) else set(args.extras.split(","))
     workloads, lat, part = {}, None, None
-    sub_steps, sub_warm = max(3, min(args.steps, 20)), max(3, min(args.warmup, 3))
+    sub_steps, sub_warm = args.steps, max(3, min(args.warmup, 3))
 
     def sub_leg(k2, p, c, lo_, hi_, my_group_, idx_, rr_):
         lg = Leg(k2, p, wl, args, world, rank, local_rank, c, my_group_, lo_, hi_, idx_, rr_)

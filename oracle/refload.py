@@ -1,9 +1,10 @@
-"""Import the reference's OWN hot-path modules unmodified (TEST INFRASTRUCTURE; build container only).
+"""Import the reference's OWN hot-path modules unmodified (TEST INFRASTRUCTURE, fixture generation only).
 
-/root/reference does not exist on the GPU box, so this loader is used ONLY by tests/golden/make_golden.py (to produce the
-committed fixtures) and by the not-gpu parity tests, which skip when the tree is absent.  Packages that cannot be
-installed offline are stubbed in sys.modules (SURVEY.md Appendix D): rank_bm25 -> oracle/rank_bm25_port.py,
-qdrant_client -> a NumPy exact-cosine stand-in, langchain / langgraph -> empty shells.
+The reference tree is not part of this repository: ``SENTIO_REFERENCE_ROOT`` points at a checkout of chernistry/sentio.
+This loader is used ONLY by tests/golden/make_golden.py to produce the committed fixtures; the tests themselves read the
+fixtures and never the reference.  Packages that cannot be installed offline are stubbed in sys.modules (SURVEY.md
+Appendix D): rank_bm25 -> oracle/rank_bm25_port.py, qdrant_client -> a NumPy exact-cosine stand-in, langchain /
+langgraph -> empty shells.
 """
 from __future__ import annotations
 
@@ -13,19 +14,7 @@ import types
 
 import numpy as np
 
-_REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def _pick_root() -> str:
-    """/root/reference in the build container; on the GPU box the git-ignored (but shipped) snapshot baseline/_ref that
-    ``__graft_entry__.build()`` takes from it (SURVEY.md section 7 step 1) -- never committed, never product."""
-    for cand in (os.environ.get("SENTIO_REFERENCE_ROOT"), "/root/reference", os.path.join(_REPO, "baseline", "_ref")):
-        if cand and os.path.isdir(os.path.join(cand, "src", "core", "retrievers")):
-            return cand
-    return os.environ.get("SENTIO_REFERENCE_ROOT", "/root/reference")
-
-
-REFERENCE_ROOT = _pick_root()
+REFERENCE_ROOT = os.environ.get("SENTIO_REFERENCE_ROOT", "")
 
 
 def available() -> bool:
@@ -85,7 +74,7 @@ def load():
     if _loaded is not None:
         return _loaded
     if not available():
-        raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT!r}: set SENTIO_REFERENCE_ROOT")
     from . import rank_bm25_port
 
     if "rank_bm25" not in sys.modules:

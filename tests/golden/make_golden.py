@@ -1,6 +1,7 @@
 """Generate the committed golden fixtures by EXECUTING THE REFERENCE'S OWN MODULES (build container only).
 
-    python tests/golden/make_golden.py        # needs /root/reference; writes tests/golden/*.json
+    SENTIO_REFERENCE_ROOT=<checkout of chernistry/sentio> python tests/golden/make_golden.py [fixture ...]
+                                              # writes tests/golden/<fixture>.json (default: all of them)
 
 The reference's tests hold no numeric known answers for this path (SURVEY.md section 4), so the fixtures are outputs of
 the unmodified reference code: HybridRetriever (src/core/retrievers/hybrid.py), BM25Retriever
@@ -373,11 +374,79 @@ def selector_cases(ns):
     return cases
 
 
-def main():
+def reference_nodes_cases(ns):
+    """The reference's retriever / reranker graph nodes (nodes.py:37-227), unmodified, driving THIS repository's
+    HybridRetriever and B200Reranker on the oracle-backed engine double: the node outputs are what
+    tests/test_reference_nodes.py holds the classes to."""
+    sys.path.insert(0, os.path.dirname(HERE))
+    from oracle_engine import OracleEngine
+    from test_hybrid_e2e import _OracleStore
+
+    import sentio_b200.retrievers.sparse as sparse_mod
+    from sentio_b200.cross_encoder import CrossEncoderWeights
+    from sentio_b200.document import Document
+    from sentio_b200.rerankers.b200_reranker import B200Reranker
+    from sentio_b200.retrievers.dense import DenseRetriever
+    from sentio_b200.retrievers.hybrid import HybridRetriever
+    from src.core.graph.nodes import create_reranker_node, create_retriever_node
+    from src.core.graph.state import create_initial_state
+
+    sparse_mod.B200Engine = lambda device=0: OracleEngine()
+    os.environ.pop("BM25_VARIANT", None)
+    dim, ce_seed, seq_len = 48, 3, 48
+    texts = [f"topic{i % 9} w{i % 13} w{(i * 7) % 31} alpha{i % 5} chunk number {i}" for i in range(240)]
+    ids = [f"doc-{i}" for i in range(len(texts))]
+    queries = ["topic3 w4 alpha2", "w7 chunk", "nothing-in-the-vocabulary", "topic8 topic8 w30"]
+    ce_cfg = dict(vocab_size=30522, hidden=128, layers=2, heads=4, intermediate=256, max_pos=64, type_vocab=2,
+                  ln_eps=1e-12)
+    emb = HashEmbedder(dim)
+    payloads = [{"content": t, "metadata": {"source": f"s{i % 4}", "page": i}} for i, t in enumerate(texts)]
+    store = _OracleStore(np.asarray(emb.embed_many_sync(texts), dtype=np.float32), ids, payloads)
+    corpus = [Document(id=i, text=t, metadata={"source": "corpus"}) for i, t in zip(ids, texts)]
+    eng = OracleEngine()
+    hr = HybridRetriever(dense_retriever=DenseRetriever(client=store, embedder=emb, collection_name="Sentio_docs"),
+                         sparse_retriever=sparse_mod.BM25Retriever(documents=corpus), rrf_k=60, scorer_plugins=[],
+                         fusion_method="rrf", engine=eng)
+    rr = B200Reranker(weights=CrossEncoderWeights.random(ce_cfg, seed=ce_seed), engine=eng, seq_len=seq_len)
+    retrieve_node = create_retriever_node(hr, top_k=10)
+    rerank_node = create_reranker_node(rr, top_k=4)
+
+    def docs(lst):
+        return [[d.id, d.text, dict(d.metadata)] for d in lst]
+
+    cases = []
+    for q in queries:
+        state = retrieve_node(create_initial_state(q))
+        case = dict(query=q, retrieved=docs(state["retrieved_documents"]), retrieve_metadata=dict(state["metadata"]))
+        st5 = create_initial_state(q)
+        st5["metadata"]["user_top_k"] = 5
+        case["retrieved_user_top_k_5"] = [d.id for d in retrieve_node(st5)["retrieved_documents"]]
+        state = rerank_node(state)
+        case["reranked"] = docs(state["reranked_documents"])
+        case["rerank_metadata"] = dict(state["metadata"])
+        cases.append(case)
+
+    class Boom:
+        def retrieve(self, query, top_k=10):
+            raise RuntimeError("index offline")
+
+    raising = create_retriever_node(Boom(), top_k=3)(create_initial_state("q"))
+    empty = rerank_node(create_initial_state("q"))
+    return dict(dim=dim, texts=texts, ids=ids, payloads=payloads, ce_config=ce_cfg, ce_seed=ce_seed, seq_len=seq_len,
+                retrieve_top_k=10, rerank_top_k=4, cases=cases,
+                raising_retriever=dict(error="index offline", metadata=dict(raising["metadata"]),
+                                       retrieved=docs(raising["retrieved_documents"])),
+                no_documents=dict(metadata=dict(empty["metadata"]), reranked=docs(empty["reranked_documents"])))
+
+
+FIXTURES = dict(fusion=fusion_cases, bm25=bm25_cases, scorers=scorer_cases, hybrid_e2e=hybrid_e2e_cases,
+                hybrid_cache=hybrid_cache_cases, rerank_flow=rerank_flow_cases, selector=selector_cases,
+                reference_nodes=reference_nodes_cases)
+
+
+def main(names=None):
     ns = refload.load()
-    fixtures = dict(fusion=fusion_cases(ns), bm25=bm25_cases(ns), scorers=scorer_cases(ns),
-                    hybrid_e2e=hybrid_e2e_cases(ns), hybrid_cache=hybrid_cache_cases(ns),
-                    rerank_flow=rerank_flow_cases(ns), selector=selector_cases(ns))
+    fixtures = {name: FIXTURES[name](ns) for name in (names or FIXTURES)}
     for name, data in fixtures.items():
         path = os.path.join(HERE, f"{name}.json")
         with open(path, "w") as f:
@@ -386,4 +455,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1:])

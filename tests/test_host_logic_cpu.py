@@ -261,9 +261,16 @@ def test_library_path_override(monkeypatch, tmp_path):
 
     default = lib.LIB_PATH
     assert default.name == "libsentio_b200.so" and default.parent.name == "sentio_b200"
+    # a reload rebinds the module's ctypes classes (SbCeConfig) and drops the loaded library, while engine.py keeps the
+    # classes it imported: put the original namespace back so later engines in this process still match their prototypes
+    saved = dict(vars(lib))
     monkeypatch.setenv("SENTIO_B200_LIB", str(tmp_path / "libsentio_b200_x.so"))
     try:
         assert importlib.reload(lib).LIB_PATH == tmp_path / "libsentio_b200_x.so"
     finally:
         monkeypatch.delenv("SENTIO_B200_LIB")
-        assert importlib.reload(lib).LIB_PATH == default
+        try:
+            assert importlib.reload(lib).LIB_PATH == default
+        finally:
+            vars(lib).clear()
+            vars(lib).update(saved)
