@@ -97,7 +97,7 @@ int sb_profile_read(sb_ctx* ctx, int kernel_id, int64_t* n_out, double* ms_out);
 int sb_dense_load(sb_ctx* ctx, int slot, const void* vecs, int64_t n, int32_t d, int32_t dtype, int64_t id_base);
 /*
  * Scan selection: 0 = auto (batches of >= 16 queries use the tcgen05 batched-query scan, smaller ones the CUDA-core
- * scan), 1 = CUDA-core scan only, 2 = tcgen05 scan whenever eligible.  Results are identical in every mode.
+ * scan), 1 = CUDA-core scan only; any other mode is SB_ERR_ARG.  Results are identical in both modes.
  */
 int sb_dense_set_mode(sb_ctx* ctx, int mode);
 int64_t sb_dense_count(sb_ctx* ctx, int slot);

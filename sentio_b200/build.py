@@ -45,46 +45,20 @@ def _digest(paths) -> str:
     return h.hexdigest()
 
 
-def build_variant(name: str, defines, verbose: bool = False) -> Path:
-    """A second library `libsentio_b200_<name>.so` from the same sources with extra -D flags (kernel A/B measurements;
-    loaded with SENTIO_B200_LIB=<path>)."""
+def _sources() -> list[Path]:
+    return [CSRC / s for s in SOURCES if (CSRC / s).exists()]
+
+
+def _compile_and_link(out: Path, obj_dir: Path, defines=(), verbose: bool = False) -> Path:
+    """Compile every source into obj_dir with NVCC_FLAGS plus one -D flag per entry of `defines`, link them into `out`."""
     nvcc = _nvcc()
-    out = PKG / f"libsentio_b200_{name}.so"
-    obj_dir = PKG / f"build_{name}"
     obj_dir.mkdir(exist_ok=True)
-    srcs = [CSRC / s for s in SOURCES if (CSRC / s).exists()]
+    srcs = _sources()
     flags = [*NVCC_FLAGS, *[f"-D{d}" for d in defines]]
 
     def compile_one(src: Path) -> Path:
         obj = obj_dir / (src.stem + ".o")
-        r = subprocess.run([nvcc, *flags, "-c", str(src), "-o", str(obj)], capture_output=True, text=True)
-        if r.returncode != 0:
-            raise RuntimeError(f"nvcc failed for {src.name}:\n{r.stdout}\n{r.stderr}")
-        return obj
-
-    with ThreadPoolExecutor(max_workers=min(8, len(srcs))) as ex:
-        objs = list(ex.map(compile_one, srcs))
-    link = [nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", str(out), *map(str, objs),
-            "-Xlinker", "--exclude-libs=ALL", "-lcudart_static", "-ldl", "-lrt", "-lpthread"]
-    r = subprocess.run(link, capture_output=True, text=True)
-    if r.returncode != 0:
-        raise RuntimeError(f"link failed:\n{r.stdout}\n{r.stderr}")
-    return out
-
-
-def build(force: bool = False, verbose: bool = False) -> Path:
-    srcs = [CSRC / s for s in SOURCES if (CSRC / s).exists()]
-    deps = srcs + sorted(CSRC.glob("*.cuh")) + [PKG.parent / "include" / "sentio_b200.h"]
-    stamp = OBJ / "stamp.txt"
-    digest = _digest(deps)
-    if not force and OUT.exists() and stamp.exists() and stamp.read_text() == digest:
-        return OUT
-    OBJ.mkdir(exist_ok=True)
-    nvcc = _nvcc()
-
-    def compile_one(src: Path) -> Path:
-        obj = OBJ / (src.stem + ".o")
-        cmd = [nvcc, *NVCC_FLAGS, "-c", str(src), "-o", str(obj)]
+        cmd = [nvcc, *flags, "-c", str(src), "-o", str(obj)]
         if verbose:
             cmd.insert(1, "-Xptxas=-v")
             print(" ".join(cmd), flush=True)
@@ -97,11 +71,27 @@ def build(force: bool = False, verbose: bool = False) -> Path:
 
     with ThreadPoolExecutor(max_workers=min(8, len(srcs))) as ex:
         objs = list(ex.map(compile_one, srcs))
-    link = [nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", str(OUT), *map(str, objs),
+    link = [nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", str(out), *map(str, objs),
             "-Xlinker", "--exclude-libs=ALL", "-lcudart_static", "-ldl", "-lrt", "-lpthread"]
     r = subprocess.run(link, capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError(f"link failed:\n{r.stdout}\n{r.stderr}")
+    return out
+
+
+def build_variant(name: str, defines, verbose: bool = False) -> Path:
+    """A second library `libsentio_b200_<name>.so` from the same sources with extra -D flags (kernel A/B measurements;
+    loaded with SENTIO_B200_LIB=<path>)."""
+    return _compile_and_link(PKG / f"libsentio_b200_{name}.so", PKG / f"build_{name}", defines, verbose)
+
+
+def build(force: bool = False, verbose: bool = False) -> Path:
+    deps = _sources() + sorted(CSRC.glob("*.cuh")) + [PKG.parent / "include" / "sentio_b200.h"]
+    stamp = OBJ / "stamp.txt"
+    digest = _digest(deps)
+    if not force and OUT.exists() and stamp.exists() and stamp.read_text() == digest:
+        return OUT
+    _compile_and_link(OUT, OBJ, verbose=verbose)
     stamp.write_text(digest)
     return OUT
 

@@ -1,6 +1,5 @@
 // api.cu -- context lifetime + error plumbing of libsentio_b200.
 #include <stdarg.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -44,12 +43,6 @@ int sb_create(int device, sb_ctx** out) {
   ctx->device = device;
   ctx->num_sms = prop.multiProcessorCount;
   ctx->smem_optin = prop.sharedMemPerBlockOptin;
-  // tuning knobs for experiments (bench / profiling); the defaults are the measured best
-  if (const char* v = getenv("SB_DENSE_PAIR")) ctx->dense_pair = atoi(v) != 0;
-  if (const char* v = getenv("SB_DENSE_SAMPLE")) ctx->dense_sample_per_cta = atoi(v) > 0 ? atoi(v) : 2;
-  if (const char* v = getenv("SB_DENSE_MULTISAMPLE")) ctx->dense_multisample = atoi(v) != 0;
-  if (const char* v = getenv("SB_DENSE_PREFETCH")) ctx->dense_prefetch = atoi(v) > 0 ? atoi(v) : 0;
-  if (const char* v = getenv("SB_DENSE_STAGES")) ctx->dense_max_stages = atoi(v) >= 3 ? atoi(v) : 8;
   cudaError_t se = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking);
   if (se != cudaSuccess) {
     sb_set_error("sb_create: cudaStreamCreate failed: %s", cudaGetErrorString(se));

@@ -15,7 +15,6 @@
 // memory (bm25_range_kernel below), nothing of size N is ever written or re-read in HBM / L2 (DESIGN.md K2).
 #include <algorithm>
 #include <type_traits>
-#include <stdlib.h>
 #include <string.h>
 #include <utility>
 #include <vector>
@@ -685,9 +684,8 @@ static int bm25_install_build(Bm25Index& nx, const uint16_t* tf_dev, const int32
     SB_CUDA(cudaGetLastError());
   }
   SB_CUDA(cudaStreamSynchronize(st));
-  // dense ratio rows of the head terms (df >= n_docs / 4): at most 64 rows and 2 GB; env SB_BM25_DENSE=0 disables them
-  const char* dz = getenv("SB_BM25_DENSE");
-  if (nx.n_terms > 0 && nx.n_docs >= 4096 && !(dz && atoi(dz) == 0)) {
+  // dense ratio rows of the head terms (df >= n_docs / 4): at most 64 rows and 2 GB
+  if (nx.n_terms > 0 && nx.n_docs >= 4096) {
     std::vector<int64_t> indptr_h((size_t)nx.n_terms + 1);
     SB_CUDA(cudaMemcpy(indptr_h.data(), nx.indptr, indptr_h.size() * 8, cudaMemcpyDeviceToHost));
     std::vector<std::pair<int64_t, int32_t>> heavy;   // (df, term)

@@ -574,16 +574,6 @@ ce_gemm_ws_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
         __syncwarp();
         // drain: four 64-byte row segments (32 fp16 columns each) per instruction, 8 bytes per lane.  A half-warp reads
         // rows (r, r + 4): 4 x 80 B = 80 words = 16 mod 32, so its two 64-byte segments fall on disjoint banks.
-#ifdef SB_CE_DRAIN32   // the previous drain (two rows per instruction, 4 bytes per lane), kept for A/B builds
-#pragma unroll 4
-        for (int r = 0; r < 32; r += 2) {
-          const int rr = r + sub, row = row0 + rr;
-          if (row < M) {
-            const uint32_t x = *reinterpret_cast<const uint32_t*>(st + (size_t)rr * kStageRow + (size_t)c16 * 4);
-            *reinterpret_cast<uint32_t*>(out16 + (size_t)row * N + col0 + 2 * c16) = x;
-          }
-        }
-#else
         const int c8 = lane & 7, rsel = lane >> 3;
         const int rmap = (rsel & 1) * 4 + (rsel >> 1);   // {0, 4, 1, 5}
 #pragma unroll
@@ -594,7 +584,6 @@ ce_gemm_ws_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
             *reinterpret_cast<uint2*>(out16 + (size_t)row * N + col0 + 4 * c8) = x;
           }
         }
-#endif
         __syncwarp();
       }
     }

@@ -131,13 +131,8 @@ struct sb_ctx {
   CeModel* enc = nullptr;  // query / document embedder (sb_enc_load)
   CeDocTokens* ce_tokens = nullptr;
   Bm25Build* bm25_build = nullptr;  // GPU index build in progress (sb_bm25_build_tokens .. sb_bm25_build_finish)
-  int dense_mode = 0;  // 0 = auto, 1 = CUDA-core scan only, 2 = tcgen05 batched scan whenever eligible
-  int dense_pair = 1;  // 1 = groups of > 64 queries use the cta_group::2 pair kernel (env SB_DENSE_PAIR=0 disables)
-  int dense_sample_per_cta = 2;  // tiles per CTA of the sampling pass (env SB_DENSE_SAMPLE)
+  int dense_mode = 0;  // 0 = auto, 1 = CUDA-core scan only
   int max_clusters2 = 0;  // co-resident 2-CTA clusters of the pair kernel (0 = not queried yet)
-  int dense_multisample = 1;   // the pair groups of a batch share one sampling launch (env SB_DENSE_MULTISAMPLE=0: one per group)
-  int dense_prefetch = 0;      // boxes prefetched into L2 beyond the ring (env SB_DENSE_PREFETCH; 0 = off)
-  int dense_max_stages = 8;    // cap on the TMA ring depth (env SB_DENSE_STAGES)
   // bookkeeping: kernels launched by this library, optional per-kernel CUDA-event timing (bench.py roofline leg)
   uint64_t launches = 0;
   bool prof_on = false;

@@ -1134,9 +1134,7 @@ int sb_ce_load(sb_ctx* ctx, const float* weights, int64_t n_floats, const sb_ce_
   int rc = ce_load_model(ctx, weights, n_floats, cfg, &m);
   if (rc) return rc;
   if (ctx->ce) ce_model_free(ctx->ce);
-  // the reranker runs on the fp16 residual stream (env SB_CE_FP32_STREAM=1 keeps the fp32 stream for A/B measurements)
-  const char* keep32 = getenv("SB_CE_FP32_STREAM");
-  m->fp16_stream = !(keep32 && atoi(keep32) != 0);
+  m->fp16_stream = true;   // the reranker runs on the fp16 residual stream (see CeModel::fp16_stream)
   ctx->ce = m;
   return SB_OK;
 }

@@ -996,7 +996,7 @@ int sb_dense_load(sb_ctx* ctx, int slot, const void* vecs, int64_t n, int32_t d,
 }
 
 int sb_dense_set_mode(sb_ctx* ctx, int mode) {
-  SB_REQUIRE(ctx != nullptr && mode >= 0 && mode <= 2, SB_ERR_ARG, "sb_dense_set_mode: bad arguments");
+  SB_REQUIRE(ctx != nullptr && (mode == 0 || mode == 1), SB_ERR_ARG, "sb_dense_set_mode: bad arguments");
   std::lock_guard<std::mutex> lk(ctx->mu);
   ctx->dense_mode = mode;
   return SB_OK;

@@ -40,6 +40,8 @@ constexpr int kTileRows = 128;
 constexpr int kBK = 64;                       // fp16 elements per 128-byte swizzle row
 constexpr uint32_t kATileBytes = kTileRows * kBK * 2;   // 16 KB
 constexpr int kMmaThreads = 192;
+constexpr int kMaxStages = 8;                 // cap on the TMA ring depth of the scan kernels
+constexpr int kSampleTilesPerCta = 2;         // least corpus tiles per CTA of the sampling pass
 constexpr int kSelectThreads = 512;
 constexpr int kSelStage = 8192;               // survivors staged in shared memory by dense_select_kernel (64 KB)
 constexpr int kSelTop = 2048;                 // window (winner) buffer; larger windows go to the exact fallback
@@ -49,10 +51,6 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map
       "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(dst),
       "l"(map), "r"(c0), "r"(c1), "r"(bar)
       : "memory");
-}
-// L2 prefetch of a tensor-map box (no shared-memory destination): keeps more HBM requests in flight than the ring holds
-__device__ __forceinline__ void tma_prefetch_l2_2d(const CUtensorMap* map, int c0, int c1) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global [%0, {%1, %2}];" ::"l"(map), "r"(c0), "r"(c1) : "memory");
 }
 
 __device__ __forceinline__ uint64_t make_smem_desc_sw128(uint32_t smem_addr) {
@@ -164,7 +162,6 @@ struct MmaScanParams {
   int32_t tile_first, tile_step; // global tile index = tile_first + t * tile_step,  t in [0, num_tiles)
   int32_t capg;
   int32_t stages;
-  int32_t prefetch;             // boxes (16 KB) prefetched into L2 beyond the shared-memory ring (0 = off)
   // pair kernel, SAMPLING pass only: n_groups query groups of 128 operand rows handled by one launch, one after the other
   // (group g: operand rows [128 g, 128 g + 128) of tm_q, lists at cand + g * group_cand_stride, counts + g * group_cnt_stride)
   int32_t n_groups;
@@ -230,17 +227,11 @@ dense_scan_mma_kernel(const __grid_constant__ CUtensorMap tm_rows, const __grid_
       mbar_expect_tx(bar_q, q_bytes);
       for (int kb = 0; kb < p.kb_count; ++kb) tma_load_2d(base + (uint32_t)kb * kQBlockBytes, &tm_q, kb * kBK, 0, bar_q);
       int it = 0;
-      const int total_it = my_tiles * p.kb_count;
       for (int t = 0; t < my_tiles; ++t) {
         const int tile = p.tile_first + (cta + t * grid) * p.tile_step;
         for (int kb = 0; kb < p.kb_count; ++kb, ++it) {
           const int s = it % p.stages;
           const uint32_t use = (uint32_t)(it / p.stages);
-          const int pf = it + p.stages + p.prefetch;   // a box the ring will only reach later: pull it into L2 now
-          if (p.prefetch > 0 && pf < total_it) {
-            const int pt = pf / p.kb_count, pkb = pf - pt * p.kb_count;
-            tma_prefetch_l2_2d(&tm_rows, pkb * kBK, (p.tile_first + (cta + pt * grid) * p.tile_step) * kTileRows);
-          }
           if (it >= p.stages) mbar_wait(bar_empty + 8 * s, (use & 1u) ^ 1u);
           mbar_expect_tx(bar_full + 8 * s, kATileBytes);
           tma_load_2d(a0 + (uint32_t)s * kATileBytes, &tm_rows, kb * kBK, tile * kTileRows, bar_full + 8 * s);
@@ -395,7 +386,6 @@ dense_scan_mma2_kernel(const __grid_constant__ CUtensorMap tm_rows, const __grid
     if (lane == 0) {
       const uint32_t lead_q = mapa_u32(bar_q, 0);
       int it = 0;
-      const int total_it = my_tiles * p.kb_count;
       for (int g = 0; g < n_groups; ++g) {
       // the query operand of group g replaces that of group g - 1 once every MMA that read it has completed
       if (g > 0) mbar_wait(bar_qfree, (uint32_t)(g - 1) & 1u);
@@ -409,12 +399,6 @@ dense_scan_mma2_kernel(const __grid_constant__ CUtensorMap tm_rows, const __grid
         for (int kb = 0; kb < p.kb_count; ++kb, ++it) {
           const int s = it % p.stages;
           const uint32_t use = (uint32_t)(it / p.stages);
-          const int pf = (it - g * total_it) + p.stages + p.prefetch;   // a box the ring will only reach later: L2 prefetch
-          if (p.prefetch > 0 && pf < total_it) {
-            const int pt = pf / p.kb_count, pkb = pf - pt * p.kb_count;
-            const int pli = 2 * (pair + pt * npairs) + (int)rank;
-            if (pli < p.num_tiles) tma_prefetch_l2_2d(&tm_rows, pkb * kBK, (p.tile_first + pli * p.tile_step) * kTileRows);
-          }
           if (it >= p.stages) mbar_wait(bar_empty + 8 * s, (use & 1u) ^ 1u);
           if (rank == 0) mbar_expect_tx(bar_full + 8 * s, 2u * kATileBytes);
           tma_load_2d_pair(a0 + (uint32_t)s * kATileBytes, &tm_rows, kb * kBK, tile * kTileRows,
@@ -754,6 +738,17 @@ int pair_clusters(sb_ctx* ctx, size_t smem) {
   return n;
 }
 
+// TMA ring of a scan CTA whose query operand takes q_bytes of shared memory: as many 16 KB stages as fit, at least 3 and
+// at most kMaxStages, plus 2 KB of barriers / thresholds / counts and 1 KB of alignment slack
+struct Ring {
+  int stages;
+  size_t smem;
+};
+Ring ring_for(const sb_ctx* ctx, size_t q_bytes) {
+  const int stages = std::max(3, std::min((int)((ctx->smem_optin - q_bytes - 3072) / kATileBytes), kMaxStages));
+  return {stages, q_bytes + (size_t)stages * kATileBytes + 2048 + 1024};
+}
+
 }  // namespace
 
 bool dense_mma_eligible(const sb_ctx* ctx, const DenseIndex& ix, int B) {
@@ -772,22 +767,20 @@ int dense_mma_topk_enqueue(sb_ctx* ctx, DenseIndex& ix, const float* q_pad, int 
   int qbn_max = 64;
   while (qbn_max > 16 && (size_t)qbn_max * ix.d_pad * 2 + 3 * (size_t)kATileBytes + 4096 > ctx->smem_optin) qbn_max >>= 1;
   // the pair kernel holds 64 operand rows per CTA: usable whenever the 64-row block fits
-  const bool pair_ok = ctx->dense_pair != 0 && qbn_max == 64 && total_tiles >= 2;
+  const bool pair_ok = qbn_max == 64 && total_tiles >= 2;
   const int gsz = pair_ok ? 128 : qbn_max;          // operand rows per group
   const int grid1 = std::min(ctx->num_sms, total_tiles);
-  int grid2 = 0, stages2 = 0;
-  size_t smem2 = 0;
+  int grid2 = 0;
+  Ring ring2 = {0, 0};
   if (pair_ok) {
-    const size_t q_bytes = (size_t)64 * ix.d_pad * 2;
-    stages2 = std::max(3, std::min((int)((ctx->smem_optin - q_bytes - 3072) / kATileBytes), ctx->dense_max_stages));
-    smem2 = q_bytes + (size_t)stages2 * kATileBytes + 2048 + 1024;
-    grid2 = 2 * std::min(pair_clusters(ctx, smem2), (total_tiles + 1) / 2);
+    ring2 = ring_for(ctx, (size_t)64 * ix.d_pad * 2);
+    grid2 = 2 * std::min(pair_clusters(ctx, ring2.smem), (total_tiles + 1) / 2);
   }
   const int grid = std::max(grid1, grid2);          // list slots per query: both kernels index [row][grid][capg]
   const int grid_min = grid2 > 0 ? std::min(grid1, grid2) : grid1;
   // sampling pass geometry: a few tiles per CTA spread evenly over the corpus; every warp of a sampled tile reports the
   // best of its 32 rows, so a query gets n_s = 4 * sample_tiles keys -- aim for n_s >= 4 k
-  const int per_cta = std::max(ctx->dense_sample_per_cta, std::min(8, (k + grid - 1) / grid));
+  const int per_cta = std::max(kSampleTilesPerCta, std::min(8, (k + grid - 1) / grid));
   const int sample_tiles = std::min(per_cta * grid, total_tiles);
   const int sample_step = total_tiles / sample_tiles;
   const int sgrid1 = std::min(grid1, sample_tiles);
@@ -833,7 +826,7 @@ int dense_mma_topk_enqueue(sb_ctx* ctx, DenseIndex& ix, const float* q_pad, int 
   for (int c0 = 0; c0 < B; c0 += gmax * gsz) {
     const int nq_chunk = std::min(B - c0, gmax * gsz);   // real queries of this chunk of groups
     const int ng = (nq_chunk + gsz - 1) / gsz;
-    struct Group { int qbn, nq; bool pair; CUtensorMap tm_q; size_t smem; int stages; };
+    struct Group { int qbn, nq; bool pair; CUtensorMap tm_q; Ring ring; };
     std::vector<Group> gs((size_t)ng);
     int rows_total = 0;  // operand rows of the chunk (padding only at the very end)
     for (int g = 0; g < ng; ++g) {
@@ -845,16 +838,13 @@ int dense_mma_topk_enqueue(sb_ctx* ctx, DenseIndex& ix, const float* q_pad, int 
         G.qbn = 128;
         G.nq = std::min(128, left);
         if ((rc = encode_map(&G.tm_q, q16g, 128, ix.d_pad, 64))) return rc;   // box = one CTA's 64 operand rows
-        G.stages = stages2;
-        G.smem = smem2;
+        G.ring = ring2;
       } else {
         G.qbn = qbn_max;
         while (G.qbn > 16 && G.qbn / 2 >= left) G.qbn >>= 1;
         G.nq = std::min(G.qbn, left);
         if ((rc = encode_map(&G.tm_q, q16g, G.qbn, ix.d_pad, G.qbn))) return rc;
-        const size_t q_bytes = (size_t)G.qbn * ix.d_pad * 2;
-        G.stages = std::max(3, std::min((int)((ctx->smem_optin - q_bytes - 3072) / kATileBytes), ctx->dense_max_stages));
-        G.smem = q_bytes + (size_t)G.stages * kATileBytes + 2048 + 1024;
+        G.ring = ring_for(ctx, (size_t)G.qbn * ix.d_pad * 2);
       }
       rows_total = g * gsz + G.qbn;
     }
@@ -863,7 +853,6 @@ int dense_mma_topk_enqueue(sb_ctx* ctx, DenseIndex& ix, const float* q_pad, int 
     mp.n = ix.n;
     mp.kb_count = kb_count;
     mp.capg = capg;
-    mp.prefetch = ctx->dense_prefetch;
     mp.n_groups = 1;
     mp.group_cand_stride = 0;
     mp.group_cnt_stride = 0;
@@ -896,30 +885,27 @@ int dense_mma_topk_enqueue(sb_ctx* ctx, DenseIndex& ix, const float* q_pad, int 
       ProfScope ps(ctx, SB_PROF_DENSE_SAMPLE, st, ng + 1);   // the sampling passes + their threshold select, as one span
       // the leading pair groups of the chunk share ONE sampling launch (a sampling launch is ~27 us of fixed cost: launch,
       // TMEM allocation, cluster syncs, the first operand load -- paid once instead of once per 128 queries)
-      int g_first = 0;
       int n_pair = 0;
       while (n_pair < ng && gs[(size_t)n_pair].pair) ++n_pair;
-      if (ctx->dense_multisample != 0 && n_pair >= 2) {
+      if (n_pair > 0) {
         CUtensorMap tm_q_all;
         if ((rc = encode_map(&tm_q_all, q16 + (size_t)c0 * ix.d_pad, (int64_t)n_pair * 128, ix.d_pad, 64))) return rc;
         mp.cand = cand;
         mp.counts = counts;
-        mp.stages = stages2;
+        mp.stages = ring2.stages;
         mp.n_groups = n_pair;
         mp.group_cand_stride = (int64_t)gsz * sgrid * capg;
         mp.group_cnt_stride = (int64_t)gsz * sgrid;
-        if ((rc = launch_mma_pair(tm_rows, tm_q_all, mp, sgrid, smem2, st))) return rc;
+        if ((rc = launch_mma_pair(tm_rows, tm_q_all, mp, sgrid, ring2.smem, st))) return rc;
         mp.n_groups = 1;
-        g_first = n_pair;
       }
-      for (int g = g_first; g < ng; ++g) {
+      // the single-CTA groups: all of them without the pair kernel, else only a trailing group of <= 64 queries
+      for (int g = n_pair; g < ng; ++g) {
         const Group& G = gs[(size_t)g];
         mp.cand = cand + (size_t)g * gsz * sgrid * capg;
         mp.counts = counts + (size_t)g * gsz * sgrid;
-        mp.stages = G.stages;
-        if (G.pair) rc = launch_mma_pair(tm_rows, G.tm_q, mp, sgrid, G.smem, st);
-        else rc = dispatch_mma(G.qbn, tm_rows, G.tm_q, mp, sgrid, G.smem, st);
-        if (rc) return rc;
+        mp.stages = G.ring.stages;
+        if ((rc = dispatch_mma(G.qbn, tm_rows, G.tm_q, mp, sgrid, G.ring.smem, st))) return rc;
       }
       sp.grid = sgrid;
       sp.mode = 0;
@@ -936,10 +922,10 @@ int dense_mma_topk_enqueue(sb_ctx* ctx, DenseIndex& ix, const float* q_pad, int 
       mp.fallback = fb + c0 + (size_t)g * gsz;
       mp.cand = cand + (size_t)g * gsz * grid * capg;
       mp.counts = counts + (size_t)g * gsz * grid;
-      mp.stages = G.stages;
+      mp.stages = G.ring.stages;
       ProfScope ps(ctx, SB_PROF_DENSE_SCAN, st);
-      if (G.pair) rc = launch_mma_pair(tm_rows, G.tm_q, mp, grid, G.smem, st);
-      else rc = dispatch_mma(G.qbn, tm_rows, G.tm_q, mp, grid, G.smem, st);
+      if (G.pair) rc = launch_mma_pair(tm_rows, G.tm_q, mp, grid, G.ring.smem, st);
+      else rc = dispatch_mma(G.qbn, tm_rows, G.tm_q, mp, grid, G.ring.smem, st);
       if (rc) return rc;
     }
     sp.grid = grid;

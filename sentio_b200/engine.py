@@ -101,7 +101,7 @@ class B200Engine:
         self.dense_count[slot] = n
 
     def dense_set_mode(self, mode: int) -> None:
-        """0 = auto, 1 = CUDA-core scan only, 2 = tcgen05 batched scan whenever eligible."""
+        """0 = auto (batches of >= 16 queries use the tcgen05 batched scan when eligible), 1 = CUDA-core scan only."""
         check(self._lib.sb_dense_set_mode(self._h, int(mode)), "sb_dense_set_mode")
 
     def pinned_empty(self, shape, dtype) -> np.ndarray:

@@ -76,3 +76,15 @@ def test_product_never_imports_the_oracle():
             if fn.endswith((".py", ".cu", ".cuh")):
                 src = open(os.path.join(dirpath, fn)).read()
                 assert not re.search(r"^\s*(from|import)\s+oracle\b", src, flags=re.M), f"{fn} imports oracle/"
+
+
+def test_library_has_no_ab_switches():
+    """Kernel A/B runs on a second build (`python -m sentio_b200.build --variant`, loaded with SENTIO_B200_LIB): the
+    library's sources read no environment variable and keep no alternative code behind an SB_ macro."""
+    switch = re.compile(r"^\s*#\s*(ifdef|ifndef)\s+SB_|^\s*#\s*(el)?if\b.*\bdefined\s*\(?\s*SB_", flags=re.M)
+    csrc = os.path.join(ROOT, "sentio_b200", "csrc")
+    for fn in sorted(os.listdir(csrc)):
+        if fn.endswith((".cu", ".cuh")):
+            src = open(os.path.join(csrc, fn)).read()
+            assert "getenv" not in src, f"{fn} reads the environment"
+            assert not switch.search(src), f"{fn} compiles code behind an SB_ macro"

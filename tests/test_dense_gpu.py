@@ -52,6 +52,16 @@ def test_dense_batched_tcgen05_path_matches_oracle(engine, n, d, k, B):
     assert np.array_equal(ids, ids1) and np.array_equal(sc, sc1) and np.array_equal(cnt, cnt1)
 
 
+def test_dense_set_mode_accepts_only_auto_and_cuda_core(engine):
+    from sentio_b200._lib import SentioB200Error
+
+    for mode in (-1, 2):
+        with pytest.raises(SentioB200Error):
+            engine.dense_set_mode(mode)
+    engine.dense_set_mode(1)
+    engine.dense_set_mode(0)
+
+
 def _near_tie_corpus(rng, n, d, cluster, ulps=1):
     """Random unit corpus whose rows [200, 200+cluster) are 1-ulp (fp16) perturbations of one base row: their cosines
     with any query differ by ~1e-6 .. 1e-5, far below the fp16-query rounding error of the tcgen05 scan."""
